@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the NeuralUDF volume-rendering hot path (BASELINE.json metric: ray-samples/s, render_core fwd+bwd).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[1], "C2" in SURVEY.md 8(d)): 512 rays x 128 uniform samples per GPU, UDF 8x256 +
 ResidualRenderingNetwork 2x(4x128) (reference conf dims), synthetic seeded sphere scene.  One step = what one training
@@ -21,6 +21,9 @@ Prints ONE JSON line (rank 0):
   workloads  the other BASELINE.json configs (C1 forward, C3 blending step, C4 whole training step incl. strong-scaling size,
              C5 256^3 grid sweep) so that the driver records them as well.
 `--impl reference` times the same CPU arm alone; under torchrun only rank 0 works.
+`--dump-outputs DIR` writes what the last timed C2 step computed (render_core outputs, loss, parameter gradients and the
+parameters after the Adam update) as DIR/<name>.npy, so that two builds can be compared output for output on identical
+seeded inputs.
 """
 import argparse
 import ctypes
@@ -245,6 +248,30 @@ def read_families(lib, n_steps, ms_step, P, pk):
     return fam
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, ret, loss, named_modules):
+    """rank 0: every tensor the caller of the timed step receives, as float32 (float64 stays float64) .npy files."""
+    arrays = {"loss": loss}
+    arrays.update(("out." + k, v) for k, v in ret.items() if isinstance(v, torch.Tensor))
+    for mname, m in named_modules:
+        for pname, p in m.named_parameters():
+            arrays["param.%s.%s" % (mname, pname)] = p
+            if p.grad is not None:
+                arrays["grad.%s.%s" % (mname, pname)] = p.grad
+    arrays = {k: v.detach().to("cpu", torch.float64 if v.dtype == torch.float64 else torch.float32).contiguous().numpy()
+              for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    return total
+
+
 def run_ours(args):
     import torch.distributed as dist
     from neuraludf_b200 import _lib
@@ -279,11 +306,17 @@ def run_ours(args):
     bucket = GradBucket(params, modules=(udf, col))      # backward kernels write dg / dv / db straight into the flat bucket
     opt = make_optimizer(udf, (col, var, beta))
 
+    # outputs of the latest step (inside a graph: its static tensors), detached: a reference into the autograd graph of an
+    # eager step would keep its AccumulateGrad nodes alive into the capture on the side stream and invalidate the capture
+    last = {}
+
     def compute(o_, d_, z_):
         opt.zero_grad(set_to_none=True)
         ret = ren.render_core(o_, d_, z_, sd, udf, var, col, beta_network=beta, cos_anneal_ratio=0.5)
         loss = loss_fn(ret, tgt)
         loss.backward()
+        last["ret"] = {k: v.detach() if isinstance(v, torch.Tensor) else v for k, v in ret.items()}
+        last["loss"] = loss.detach()
         return loss
 
     def step(o_, d_, z_):
@@ -373,6 +406,9 @@ def run_ours(args):
         clocks.end()
     ms = e0.elapsed_time(e1)
     clk = clocks.stop() if clocks else None
+    if args.dump_outputs and rank == 0:               # before any further step changes the parameters
+        dump_outputs(args.dump_outputs, last["ret"], last["loss"],
+                     (("udf", udf), ("color", col), ("variance", var), ("beta", beta)))
 
     if args.quick:
         if rank == 0:
@@ -806,7 +842,14 @@ def main():
                     "family table, no CPU baseline, no secondary workloads; prints a reduced JSON line")
     ap.add_argument("--no-extra", dest="no_extra", action="store_true", help="skip the secondary workloads")
     ap.add_argument("--no-graph", dest="no_graph", action="store_true", help="time the eager loop only (no CUDA-graph capture)")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed C2 step (render_core outputs, loss, parameter gradients, "
+                         "updated parameters) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "c2"):
+        ap.error("--dump-outputs applies to the C2 workload of --impl ours")
     out = run_reference(args) if args.impl == "reference" else run_ours(args)
     if out is not None:
         print(json.dumps(out), flush=True)

@@ -192,5 +192,75 @@ static inline int run_fold_jobs(const FoldJobs& jobs, bool unfold, cudaStream_t 
   return 0;
 }
 
+// ---- deterministic split reductions --------------------------------------------------------------------------------------------
+// A contraction split over CTAs (split-K over points) writes each split's partial result into its own slice of a stream-ordered
+// workspace; sum_slices then adds the slices to the destination in a fixed order.  Float atomics would add the partials in
+// whatever order the CTAs finish, so the weight gradients -- and every training step after them -- would differ from run to run.
+struct SliceJob {                      // C[r, c] += sum over z of ws[z * slice + r * ldw + c],  r < rows, c < cols
+  const float* ws; int64_t slice, ldw;
+  int rows, cols;
+  float* C; int64_t ldc;
+};
+constexpr int NUDF_MAX_SLICE_JOBS = 3;
+struct SliceJobs { int n, slices; SliceJob j[NUDF_MAX_SLICE_JOBS]; };
+// grid = (elements / 32, jobs), 256 threads: lane = element, warp w sums slices w, w + 8, ... and the 8 partial sums are added
+// in warp order -- a fixed tree, whatever the scheduling.
+static __global__ void __launch_bounds__(256) sum_slices_kernel(const __grid_constant__ SliceJobs jobs) {
+  const SliceJob& J = jobs.j[blockIdx.y];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int64_t i = (int64_t)blockIdx.x * 32 + lane;
+  const bool ok = i < (int64_t)J.rows * J.cols;
+  const int64_t r = ok ? i / J.cols : 0, c = ok ? i - r * J.cols : 0;
+  float s = 0.f;
+  if (ok) {
+    const float* p = J.ws + r * J.ldw + c;
+#pragma unroll 4
+    for (int z = w; z < jobs.slices; z += 8) s += __ldcs(p + (int64_t)z * J.slice);
+  }
+  __shared__ float part[8][32];
+  part[w][lane] = s;
+  __syncthreads();
+  if (w == 0 && ok) {
+    float t = part[0][lane];
+#pragma unroll
+    for (int k = 1; k < 8; ++k) t += part[k][lane];
+    J.C[r * J.ldc + c] += t;
+  }
+}
+// status of the launch just issued (counts it like NUDF_LAUNCH_OK, but returns instead of leaving the caller's scope, so that
+// a workspace can still be released)
+static inline int launch_status() {
+  nudf::count_launch();
+  const cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess) return 0;
+  nudf::set_error("kernel launch -> %s", cudaGetErrorString(e));
+  return -2;
+}
+// workspace of `floats` floats, allocated in stream order (capturable into a CUDA graph); release with slices_free
+static inline int slices_alloc(float** ws, size_t floats, cudaStream_t st) {
+  NUDF_CUDA_OK(cudaMallocAsync((void**)ws, floats * sizeof(float), st));
+  return 0;
+}
+static inline int slices_free(float* ws, cudaStream_t st) {
+  NUDF_CUDA_OK(cudaFreeAsync(ws, st));
+  return 0;
+}
+static inline int sum_slices(const SliceJobs& jobs, cudaStream_t st) {
+  int64_t most = 0;
+  for (int k = 0; k < jobs.n; ++k) most = (int64_t)jobs.j[k].rows * jobs.j[k].cols > most ? (int64_t)jobs.j[k].rows * jobs.j[k].cols : most;
+  if (most <= 0) return 0;
+  sum_slices_kernel<<<dim3((unsigned)cdiv(most, 32), (unsigned)jobs.n), 256, 0, st>>>(jobs);
+  return launch_status();
+}
+// one destination: C[r, c] += sum over z of ws[z * slice + r * ldw + c]
+static inline int sum_slices(const float* ws, int slices, int64_t slice, int64_t ldw, int rows, int cols, float* C, int64_t ldc,
+                             cudaStream_t st) {
+  SliceJobs jobs{};
+  jobs.n = 1;
+  jobs.slices = slices;
+  jobs.j[0] = SliceJob{ws, slice, ldw, rows, cols, C, ldc};
+  return sum_slices(jobs, st);
+}
+
 }  // namespace nudf
 #endif

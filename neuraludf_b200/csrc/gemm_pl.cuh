@@ -370,6 +370,16 @@ static inline int gemm_tn_pl(const Planes& X, int M, const Planes& Y, int N, int
   if (splits < 1) splits = 1;
   const int64_t bps = cdiv(n_blocks, (int64_t)splits);
   splits = (int)cdiv(n_blocks, bps);
+  if constexpr (std::is_same<Epi, EpiAtomicAdd>::value) {     // fixed-order split-K: slices + sum_slices
+    const int64_t ldw = round_up(N, 4), slice = (int64_t)M * ldw;
+    float* ws = nullptr;
+    int rc = slices_alloc(&ws, (size_t)(slice * splits), st);
+    if (rc != 0) return rc;
+    rc = gemm_tn_pl(X, M, Y, N, P, EpiSliceStore{ws, ldw, slice}, st, splits);
+    if (rc == 0) rc = sum_slices(ws, splits, slice, ldw, M, N, epi.C, epi.ldc, st);
+    const int rf = slices_free(ws, st);
+    return rc != 0 ? rc : rf;
+  }
   const size_t smem = (size_t)TP_STAGES * TP_STAGE_BYTES + sizeof(SmemCtlT) + 1024 + 64;
   static bool attr_set = false;
   if (!attr_set) {

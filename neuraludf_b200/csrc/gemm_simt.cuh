@@ -7,8 +7,10 @@
 //     A(m,k) = A_KC ? A[m*lda + k] : A[k*lda + m]
 //     B(k,n) = B_KC ? B[n*ldb + k] : B[k*ldb + n]
 // so  X W^T (forward / tangent chains)  is <true,true>,   dY W (reverse / backward chains) is <true,false>,
-// and dY^T X (weight gradients, contraction over points, split over gridDim.z with atomics) is <false,false>.
+// and dY^T X (weight gradients, contraction over points, split over gridDim.z into ordered slices) is <false,false>.
 #pragma once
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace nudf {
@@ -218,7 +220,8 @@ struct EpiAct {
   NUDF_EPI_CALL
 };
 
-// C[row, col] += acc   (split-K partial sums of weight gradients)
+// C[row, col] += acc   (split-K partial sums of weight gradients).  The launchers run it as EpiSliceStore + sum_slices, so
+// that the partials are added in a fixed order.
 struct EpiAtomicAdd {
   float* C; int64_t ldc;
   struct Aux {};
@@ -233,6 +236,24 @@ struct EpiAtomicAdd {
 #pragma unroll
     for (int j = 0; j < 4; ++j)
       if (j < nv) atomicAdd(p + j, acc[j]);
+  }
+  NUDF_EPI_CALL
+};
+
+// (C + blockIdx.z * slice)[row, col] = acc: the partial tile of split blockIdx.z, in its own workspace slice (sum_slices)
+struct EpiSliceStore {
+  float* C; int64_t ldc; int64_t slice;
+  struct Aux {};
+  __device__ __forceinline__ void load(int64_t, int, int, Aux&) const {}
+  __device__ __forceinline__ void apply(int64_t row, int col, const float acc[4], int nv, const Aux&) const {
+    float* p = C + (int64_t)blockIdx.z * slice + row * ldc + col;
+    if (nv == 4 && ((ldc & 3) == 0) && ((slice & 3) == 0) && ((col & 3) == 0) && aligned16(C)) {
+      *reinterpret_cast<float4*>(p) = make_float4(acc[0], acc[1], acc[2], acc[3]);
+      return;
+    }
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+      if (j < nv) p[j] = acc[j];
   }
   NUDF_EPI_CALL
 };
@@ -404,6 +425,18 @@ template <bool A_KC, bool B_KC, class Epi>
 static inline int gemm_simt(const float* A, int64_t lda, const float* B, int64_t ldb, int64_t M, int N, int64_t K,
                             const Epi& epi, cudaStream_t st, int split_k = 1) {
   if (M <= 0 || N <= 0) return 0;
+  if constexpr (std::is_same<Epi, EpiAtomicAdd>::value) {     // fixed-order split-K: slices + sum_slices
+    if (K <= 0) return 0;
+    const int splits = split_k > 1 ? (int)cdiv(K, round_up(cdiv(K, split_k), GS_BK)) : 1;
+    const int64_t ldw = round_up(N, 4), slice = M * ldw;
+    float* ws = nullptr;
+    int rc = slices_alloc(&ws, (size_t)(slice * splits), st);
+    if (rc != 0) return rc;
+    rc = gemm_simt<A_KC, B_KC, EpiSliceStore>(A, lda, B, ldb, M, N, K, EpiSliceStore{ws, ldw, slice}, st, split_k);
+    if (rc == 0) rc = sum_slices(ws, splits, slice, ldw, (int)M, N, epi.C, epi.ldc, st);
+    const int rf = slices_free(ws, st);
+    return rc != 0 ? rc : rf;
+  }
   LaunchTimer lt_(FAM_FFMA, st);
   int64_t k_chunk = K;
   if (split_k > 1) {

@@ -16,7 +16,7 @@
 //   warp 9     weight loader: one lane issues cp.async.bulk (TMA engine, UBLKCP) of the pre-split, pre-swizzled weight
 //              slice image (built once per optimiser step by tc_prep_weights_kernel) with mbarrier complete_tx.
 // The weight-gradient variant (gemm_tn) stages BOTH operands from fp32 activations with an on-the-fly transpose
-// (contraction over points) and accumulates split-K partial tiles with red.global.add.
+// (contraction over points); each split-K partial tile goes to its own workspace slice, added in order by sum_slices.
 #pragma once
 #include <cuda_bf16.h>
 
@@ -827,7 +827,7 @@ gemm_wr_kernel(const float* __restrict__ A, int64_t lda, int64_t M, int N, int K
 
 // ---------------------------------------------------------------------------------------------------------------
 // C[M x N] += A[K x M]^T B[K x N]  (weight gradients; contraction over points, split over gridDim.z).
-// grid = (ceil(M/128), ceil(N/256), splits).  Epi is applied to the partial tile (EpiAtomicAdd).
+// grid = (ceil(M/128), ceil(N/256), splits).  Epi is applied to the partial tile (EpiSliceStore: slice blockIdx.z).
 // ---------------------------------------------------------------------------------------------------------------
 constexpr int TN_PROD = 384;      // 12 loading / epilogue warps: 4 stage the [128 x 64] A^T tile, 8 the [256 x 64] B^T tile
 constexpr int TN_THREADS = 416;   // + warp 12: MMA issuer and TMEM owner
@@ -891,7 +891,7 @@ gemm_tn_kernel(const float* __restrict__ A, int64_t lda, const float* __restrict
         const int m = m0 + 32 * warp + 4 * (lane & 7);
 #pragma unroll
         for (int j = 0; j < 4; ++j)
-          if (m + j < M) atomicAdd(colsum_a + m + j, csum[j]);
+          if (m + j < M) atomicAdd(colsum_a + (int64_t)blockIdx.z * M + m + j, csum[j]);   // this split's slice
       }
     }
     if (n_slices > 0) {
@@ -1012,6 +1012,26 @@ static inline int gemm_tn(const float* A, int64_t lda, const float* B, int64_t l
   if (M <= 0 || N <= 0 || K <= 0) return 0;
   int64_t k_chunk = round_up(cdiv(K, split_k < 1 ? 1 : split_k), BK);
   int splits = (int)cdiv(K, k_chunk);
+  if constexpr (std::is_same<Epi, EpiAtomicAdd>::value) {     // fixed-order split-K: slices + sum_slices
+    const int64_t ldw = round_up(N, 4), slice = (int64_t)M * ldw, cs = colsum_a ? (int64_t)splits * M : 0;
+    float* ws = nullptr;
+    int rc = slices_alloc(&ws, (size_t)(slice * splits + cs), st);
+    if (rc != 0) return rc;
+    float* wcs = colsum_a ? ws + slice * splits : nullptr;
+    if (wcs != nullptr && cudaMemsetAsync(wcs, 0, (size_t)cs * sizeof(float), st) != cudaSuccess) rc = -2;
+    if (rc == 0) rc = gemm_tn(A, lda, B, ldb, M, N, K, EpiSliceStore{ws, ldw, slice}, st, split_k, wcs, t128);
+    if (rc == 0) {
+      SliceJobs jobs{};
+      jobs.slices = splits;
+      jobs.j[jobs.n++] = SliceJob{ws, slice, ldw, M, N, epi.C, epi.ldc};
+      if (wcs != nullptr) jobs.j[jobs.n++] = SliceJob{wcs, M, M, 1, M, colsum_a, M};
+      rc = sum_slices(jobs, st);
+    }
+    const int rf = slices_free(ws, st);
+    return rc != 0 ? rc : rf;
+  } else if constexpr (!std::is_same<Epi, EpiSliceStore>::value) {
+    NUDF_REQUIRE(colsum_a == nullptr, "column sums go with a split-K reduction");
+  }
   const size_t smem = smem_bytes_for(pad16(N < 256 ? N : 256), 2);
   static bool attr_set = false;
   if (!attr_set) {
@@ -1288,6 +1308,7 @@ gemm_tn2_kernel(TnPair p0, TnPair p1, int n_pairs, int M, int N, int64_t K, int6
       mbar_arrive(&ctl->full[s]);
       if (is_a && blockIdx.y == 0 && (i == n_sl - 1 || i == total - 1)) {       // end of a pair: flush its column sums
         float* out = pair_of(i).colsum_a;
+        if (out != nullptr) out += (int64_t)blockIdx.z * M;     // this split's slice
         if (out != nullptr && RM) {                     // lanes (p, g): columns r0 + 4 (g + 4 i) + j in csum[4 i + j]; reduce over p
 #pragma unroll
           for (int j = 0; j < 8; ++j) {
@@ -1352,16 +1373,45 @@ gemm_tn2_kernel(TnPair p0, TnPair p1, int n_pairs, int M, int N, int64_t K, int6
 }
 
 // row_major: operands are plain [K, ld] row-major fp32 (ld % 4 == 0, 16-byte aligned bases); else T128 (common.cuh)
-template <class Epi>
-static inline int gemm_tn2(const TnPair* pairs, int n_pairs, int M, int N, int64_t K, const Epi& epi, cudaStream_t st, bool row_major = false) {
-  if (M <= 0 || N <= 0 || K <= 0 || n_pairs <= 0) return 0;
+static inline int tn2_splits(int M, int N, int64_t K) {
   const int tiles = (int)(cdiv(M, BM) * cdiv(N, 256));
   int splits = sm_count() / tiles;
   const int max_splits = (int)cdiv(K, 256);                  // at least 8 slices of 32 points per CTA and pair
   if (splits > max_splits) splits = max_splits;
   if (splits < 1) splits = 1;
   const int64_t k_chunk = round_up(cdiv(K, splits), 128);      // whole 128-point blocks of the T128 layout per CTA
-  splits = (int)cdiv(K, k_chunk);
+  return (int)cdiv(K, k_chunk);
+}
+
+template <class Epi>
+static inline int gemm_tn2(const TnPair* pairs, int n_pairs, int M, int N, int64_t K, const Epi& epi, cudaStream_t st, bool row_major = false) {
+  if (M <= 0 || N <= 0 || K <= 0 || n_pairs <= 0) return 0;
+  if constexpr (std::is_same<Epi, EpiAtomicAdd>::value) {     // fixed-order split-K: slices + sum_slices
+    const int splits = tn2_splits(M, N, K);
+    const int np = n_pairs > 1 ? 2 : 1;
+    const int64_t ldw = round_up(N, 4), slice = (int64_t)M * ldw, cs = (int64_t)splits * M;
+    float* ws = nullptr;
+    int rc = slices_alloc(&ws, (size_t)(slice * splits + np * cs), st);
+    if (rc != 0) return rc;
+    TnPair pp[2] = {pairs[0], pairs[np - 1]};
+    bool any_cs = false;
+    for (int p = 0; p < np; ++p)
+      if (pp[p].colsum_a != nullptr) { pp[p].colsum_a = ws + slice * splits + p * cs; any_cs = true; }
+    if (any_cs && cudaMemsetAsync(ws + slice * splits, 0, (size_t)(np * cs) * sizeof(float), st) != cudaSuccess) rc = -2;
+    if (rc == 0) rc = gemm_tn2(pp, np, M, N, K, EpiSliceStore{ws, ldw, slice}, st, row_major);
+    if (rc == 0) {
+      SliceJobs jobs{};
+      jobs.slices = splits;
+      jobs.j[jobs.n++] = SliceJob{ws, slice, ldw, M, N, epi.C, epi.ldc};
+      for (int p = 0; p < np; ++p)
+        if (pairs[p].colsum_a != nullptr) jobs.j[jobs.n++] = SliceJob{pp[p].colsum_a, M, M, 1, M, pairs[p].colsum_a, M};
+      rc = sum_slices(jobs, st);
+    }
+    const int rf = slices_free(ws, st);
+    return rc != 0 ? rc : rf;
+  }
+  const int splits = tn2_splits(M, N, K);
+  const int64_t k_chunk = round_up(cdiv(K, splits), 128);      // whole 128-point blocks of the T128 layout per CTA
   const size_t smem = (size_t)T2_PLANES + (size_t)T2_RING * T2_RAW_GRAN + sizeof(SmemCtl) + 64;
   static bool attr_set[2] = {false, false};
   if (!attr_set[row_major ? 1 : 0]) {

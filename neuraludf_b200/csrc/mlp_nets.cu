@@ -161,9 +161,10 @@ static inline int dense_small_forward(const float* X, int64_t ldx, const float* 
   return 0;
 }
 
-// Weight gradient of a narrow head (n_out <= 16: colour / density heads): dW[m, n] += sum_p dZ[p, m] X[p, n], db[m] += sum_p dZ[p, m].
+// Weight gradient of a narrow head (n_out <= 16: colour / density heads): dW[m, n] += sum_p dZ[p, m] X[p, n], db[m] += sum_p dZ[p, m];
+// the kernel writes the partial sums of point chunk blockIdx.y to slice blockIdx.y of dW ([n_out, ldw] per slice) and db.
 // Streams X once (HBM-bound) instead of padding the 3..13 output rows to a 128-wide GEMM tile.  CTA = 128 input columns x 4
-// point lanes over a 256-point chunk; the lanes' partial sums meet in shared memory, then one atomic per (m, n) per CTA.
+// point lanes over a 256-point chunk; the lanes' partial sums meet in shared memory, then one store per (m, n) per CTA.
 template <int MAXM>
 __global__ void __launch_bounds__(512)
 wgrad_small_kernel(const float* __restrict__ dZ, int64_t ldz, const float* __restrict__ X, int64_t ldx, int n_out, int n_in, int64_t P,
@@ -203,9 +204,9 @@ wgrad_small_kernel(const float* __restrict__ dZ, int64_t ldz, const float* __res
   if (ty == 0 && n < n_in) {
 #pragma unroll
     for (int m = 0; m < MAXM; ++m)
-      if (m < n_out) atomicAdd(dW + (int64_t)m * ldw + n, acc[m] + red[0][m][tx] + red[1][m][tx] + red[2][m][tx]);
+      if (m < n_out) dW[((int64_t)blockIdx.y * n_out + m) * ldw + n] = acc[m] + red[0][m][tx] + red[1][m][tx] + red[2][m][tx];
   }
-  if (db != nullptr && blockIdx.x == 0 && threadIdx.x < n_out) atomicAdd(db + threadIdx.x, bs);
+  if (db != nullptr && blockIdx.x == 0 && threadIdx.x < n_out) db[(int64_t)blockIdx.y * n_out + threadIdx.x] = bs;
 }
 
 static int wgrad(const float* dZ, int64_t ldz, const float* X, int64_t ldx, int n_out, int n_in, int64_t P, float* dW,
@@ -213,9 +214,24 @@ static int wgrad(const float* dZ, int64_t ldz, const float* X, int64_t ldx, int 
   if (n_out <= 16 && P > 0) {
     const int64_t chunk = 256;
     dim3 grid((unsigned)cdiv(n_in, 128), (unsigned)cdiv(P, chunk));
-    wgrad_small_kernel<16><<<grid, 512, 0, st>>>(dZ, ldz, X, ldx, n_out, n_in, P, chunk, dW, ldw, db);
-    NUDF_LAUNCH_OK();
-    return 0;
+    // every chunk of points writes its partial sums into its own slice; sum_slices adds them in chunk order
+    const int slices = (int)grid.y;
+    const int64_t slice = (int64_t)n_out * n_in;
+    float* ws = nullptr;
+    int rc = slices_alloc(&ws, (size_t)(slices * (slice + n_out)), st);
+    if (rc != 0) return rc;
+    float* wdb = db != nullptr ? ws + slices * slice : nullptr;
+    wgrad_small_kernel<16><<<grid, 512, 0, st>>>(dZ, ldz, X, ldx, n_out, n_in, P, chunk, ws, n_in, wdb);
+    rc = launch_status();
+    if (rc == 0) {
+      SliceJobs jobs{};
+      jobs.slices = slices;
+      jobs.j[jobs.n++] = SliceJob{ws, slice, n_in, n_out, n_in, dW, ldw};
+      if (db != nullptr) jobs.j[jobs.n++] = SliceJob{wdb, n_out, n_out, 1, n_out, db, n_out};
+      rc = sum_slices(jobs, st);
+    }
+    const int rf = slices_free(ws, st);
+    return rc != 0 ? rc : rf;
   }
   int split = (int)cdiv(P, 2048);
   EpiAtomicAdd ew{dW, ldw};

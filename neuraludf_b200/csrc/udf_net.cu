@@ -368,7 +368,7 @@ __global__ void weighted_colsum_kernel(const float* __restrict__ X, int64_t ldx,
     float t = 0.f;
 #pragma unroll
     for (int k = 0; k < 8; ++k) t += red[k][threadIdx.x & 31];
-    atomicAdd(out + c, t);
+    out[(int64_t)blockIdx.y * N + c] = t;      // this row block's slice (colsum adds the slices in order)
   }
 }
 
@@ -376,9 +376,14 @@ int colsum(const float* X, int64_t ldx, const float* w, float wscale, int64_t P,
   if (P <= 0 || N <= 0) return 0;
   int64_t rpb = 512;
   dim3 grid((unsigned)cdiv(N, 32), (unsigned)cdiv(P, rpb));
-  weighted_colsum_kernel<<<grid, 256, 0, st>>>(X, ldx, w, wscale, P, N, rpb, out, t128 ? 1 : 0);
-  NUDF_LAUNCH_OK();
-  return 0;
+  float* ws = nullptr;
+  int rc = slices_alloc(&ws, (size_t)grid.y * N, st);
+  if (rc != 0) return rc;
+  weighted_colsum_kernel<<<grid, 256, 0, st>>>(X, ldx, w, wscale, P, N, rpb, ws, t128 ? 1 : 0);
+  rc = launch_status();
+  if (rc == 0) rc = sum_slices(ws, (int)grid.y, N, N, 1, N, out, N, st);
+  const int rf = slices_free(ws, st);
+  return rc != 0 ? rc : rf;
 }
 
 // Zlast[:,0] = sgn * ob[:,0] / scale ; Zlast[:,1:] = ob[:,1:]

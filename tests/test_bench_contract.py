@@ -1,9 +1,11 @@
-"""bench.py contract, CPU-checkable part: the reference arm (`--impl reference`) prints one JSON line with the agreed keys
-on rank 0 and nothing on the other ranks."""
+"""bench.py contract: the reference arm (`--impl reference`) prints one JSON line with the agreed keys on rank 0 and nothing
+on the other ranks; `--dump-outputs` writes the outputs of the last timed step (GPU)."""
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -33,3 +35,40 @@ def test_reference_arm_json_line():
 def test_reference_arm_other_ranks_are_silent():
     r = _run({"RANK": "1", "WORLD_SIZE": "2"})
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+def test_dump_outputs_needs_the_c2_workload_and_a_step():
+    for extra in (["--impl", "reference", "--dump-outputs", "x"], ["--workload", "c5", "--dump-outputs", "x"], ["--steps", "0"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, cwd=ROOT, capture_output=True, text=True,
+                           timeout=600)
+        assert r.returncode == 2 and "error:" in r.stderr, (extra, r.stderr[-500:])
+
+
+def _dump(out, steps):
+    import numpy as np
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "1", "--quick",
+                        "--dump-outputs", str(out)], cwd=ROOT, capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-2000:]
+    return {p.stem: np.load(p) for p in out.glob("*.npy")}
+
+
+@pytest.mark.gpu
+def test_dump_outputs_writes_the_last_timed_step(tmp_path):
+    """The dump is what the timed step computed: complete, reproducible bit for bit from run to run (seeded inputs, fixed-order
+    reductions), and taken after the requested number of steps (a different --steps trains the parameters further)."""
+    import numpy as np
+    import torch
+    if not torch.cuda.is_available():
+        pytest.skip("no CUDA device")
+    arrays = _dump(tmp_path / "a", 2)
+    for k in ("loss", "out.color", "out.weights", "grad.udf.lin0.weight_v", "param.udf.lin0.weight_v", "param.beta.beta"):
+        assert k in arrays, k
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    assert arrays["out.color"].shape == (512, 3) and np.isfinite(arrays["loss"]).all()
+    assert np.abs(arrays["grad.udf.lin0.weight_v"]).max() > 0
+    again = _dump(tmp_path / "b", 2)
+    assert sorted(again) == sorted(arrays)
+    assert [k for k in arrays if not np.array_equal(arrays[k], again[k])] == []
+    longer = _dump(tmp_path / "c", 3)
+    assert not np.array_equal(longer["param.udf.lin0.weight_v"], arrays["param.udf.lin0.weight_v"])

@@ -1,58 +1,36 @@
 """Device-side grid query / near-surface cell emission (neuraludf_b200/grid.py) against the reference's own
-get_udf_normals_grid_slow (extract_mesh.py:18-105, staged copy) driven with the same network callbacks."""
-import importlib
-import os
-import sys
-
+get_udf_normals_grid_slow (extract_mesh.py:18-105) driven with the same network callbacks, stored by
+oracle/make_golden_device.py in tests/golden/device_outputs.npz (the full near-surface mask, seeded samples of the rest)."""
+import numpy as np
 import pytest
 import torch
 
-from oracle import refshim
+from tests.golden_util import load_device_golden
 from tests.gpu_util import build_modules
 
 pytestmark = pytest.mark.gpu
 
 
-def _ref_extract_mesh():
-    from tests import runner_env
-    runner_env.install_stubs()
-    if refshim.REFERENCE_ROOT not in sys.path:
-        sys.path.insert(0, refshim.REFERENCE_ROOT)
-    for k in [k for k in sys.modules if k == "extract_mesh"]:
-        del sys.modules[k]
-    return importlib.import_module("extract_mesh")
-
-
-@pytest.mark.skipif(not os.path.isfile(os.path.join(refshim.REFERENCE_ROOT, "extract_mesh.py")), reason="no staged reference copy")
 def test_grid_and_near_surface_cells_match_reference(golden):
     if not torch.cuda.is_available():
         pytest.skip("no CUDA device")
     from neuraludf_b200 import grid
+    fx = load_device_golden()
     udf = build_modules(golden, "cuda")[0]
-    N = 48
-    func = udf.udf
-
-    def func_grad(xyz):                                    # exp_runner_blending.py:767-771
-        g = udf.gradient(xyz)
-        return g / (torch.linalg.norm(g, ord=2, dim=-1, keepdim=True) + 1e-5)
-
-    em = _ref_extract_mesh()
-    # the reference mixes device-less tensors with .cuda() results and relies on the runner's global default
-    # (exp_runner_blending.py:872)
-    torch.set_default_tensor_type("torch.cuda.FloatTensor")
-    try:
-        df_ref, vec_ref, samples_ref = em.get_udf_normals_grid_slow(func, func_grad, N=N, max_batch=1 << 14)
-    finally:
-        torch.set_default_tensor_type("torch.FloatTensor")
-    df_ref, vec_ref, samples_ref = df_ref.cpu(), vec_ref.cpu(), samples_ref.cpu()
+    N = int(fx["grid_n"])
+    assert N == 48
     df, vec, samples = grid.get_udf_normals_grid_slow(udf, N=N, max_batch=1 << 15)
-    assert df.shape == df_ref.shape and vec.shape == vec_ref.shape and samples.shape == samples_ref.shape
-    assert float((samples[:, :3] - samples_ref[:, :3]).abs().max()) < 1e-6          # lattice coordinates
-    assert float((df - df_ref).abs().max()) < 1e-6                                   # same kernels, different batching
-    mask_ref = (vec_ref.abs().sum(-1) > 0)
-    mask = (vec.abs().sum(-1) > 0)
+    assert df.shape == (N, N, N) and vec.shape == (N, N, N, 3) and samples.shape == (N ** 3, 7)
+    idx = torch.from_numpy(fx["grid_idx"].astype(np.int64))
+    ref = torch.from_numpy(fx["grid_samples"])
+    assert float((samples[idx, :3] - ref[:, :3]).abs().max()) < 1e-6                # lattice coordinates
+    assert float((samples[idx, 3] - ref[:, 3]).abs().max()) < 1e-6                  # same kernels, different batching
+    assert float((samples[idx, 4:] - ref[:, 4:]).abs().max()) < 1e-4
+    mask_ref = torch.from_numpy(np.unpackbits(fx["grid_mask_bits"])[:N ** 3].astype(bool))
+    mask = (vec.abs().sum(-1) > 0).reshape(-1)
     assert torch.equal(mask, mask_ref) and int(mask.sum()) > 100                     # the same near-surface cells
-    assert float((vec - vec_ref).abs().max()) < 1e-4
+    sidx = torch.from_numpy(fx["grid_surface_idx"].astype(np.int64))
+    assert float((vec.reshape(-1, 3)[sidx] - torch.from_numpy(fx["grid_surface_vec"])).abs().max()) < 1e-4
     idx, normals = grid.near_surface_cells(udf, N)
     assert idx.numel() == int(mask.sum())
     assert float((normals.norm(dim=1) - 1).abs().max()) < 1e-4

@@ -71,6 +71,27 @@ def test_dense_forward_tc_vs_fp64(M, N, K):
     assert e2 < 5e-5, e2
 
 
+@pytest.mark.parametrize("P,n_out,n_in", [(65536, 256, 256), (20000, 257, 256), (65536, 3, 259)])
+def test_wgrad_is_bitwise_reproducible(P, n_out, n_in):
+    """The split-K partials are added in a fixed order: the same inputs give the same bits on every call, accumulating
+    into a non-zero destination as the training step does."""
+    L, lib = _lib()
+    g = torch.Generator().manual_seed(P + n_in)
+    dZd = torch.randn(P, n_out, generator=g).to(DEV)
+    Xd = torch.randn(P, n_in, generator=g).to(DEV)
+    base = torch.randn(n_out, n_in, generator=g).to(DEV)
+    for engine in (1, 0):
+        outs = []
+        for _ in range(3):
+            dW = base.clone()
+            L.check(lib.nudf_wgrad(L.ptr(dZd), n_out, L.ptr(Xd), n_in, n_out, n_in, P, L.ptr(dW), n_in, engine, L.stream_ptr()),
+                    "wgrad")
+            outs.append(dW)
+        torch.cuda.synchronize()
+        assert all(torch.equal(o, outs[0]) for o in outs[1:]), engine
+        assert not torch.equal(outs[0], base)
+
+
 @pytest.mark.parametrize("P,n_out,n_in", [(1024, 256, 256), (5000, 217, 256), (3000, 128, 259), (700, 257, 256), (4096, 256, 39)])
 def test_wgrad_tc_vs_fp64(P, n_out, n_in):
     L, lib = _lib()

@@ -1,22 +1,22 @@
 """CPU checks of the test-only runner environment (tests/runner_env.py): the HOCON-subset reader parses the reference's
-four shipped confs into the values the runner reads, the nudf modules accept those conf blocks as constructor kwargs
-(exp_runner_blending.py:125-146), and the synthetic DTU-layout dataset has the files / camera keys dataset.py loads."""
+four shipped confs (stored unmodified under tests/golden/confs) into the values the runner reads, the nudf modules accept
+those conf blocks as constructor kwargs (exp_runner_blending.py:125-146), and the synthetic DTU-layout dataset has the
+files / camera keys dataset.py loads."""
 import os
 
 import numpy as np
 import pytest
 
-from oracle import refshim
 from tests import runner_env
+from tests.golden_util import GOLDEN
 
-pytestmark = pytest.mark.skipif(not refshim.available(), reason="reference checkout / staged copy not present")
 CONFS = ["confs/udf_dtu_blending.conf", "confs/udf_dtu_blending_ft.conf", "confs/udf_garment_blending.conf",
          "confs/udf_garment_blending_ft.conf"]
 
 
 @pytest.mark.parametrize("name", CONFS)
 def test_hocon_lite_parses_reference_confs(name):
-    text = open(os.path.join(refshim.REFERENCE_ROOT, name)).read().replace("CASE_NAME", "scan24")
+    text = open(os.path.join(GOLDEN, name)).read().replace("CASE_NAME", "scan24")
     c = runner_env.ConfigFactory.parse_string(text)
     assert c["general.model_type"] == "udf"
     assert isinstance(c["general.recording"], list) and c["general.recording"][0] == "./"
@@ -45,7 +45,7 @@ def test_modules_accept_conf_blocks(name):
     """exp_runner_blending.py:125-146 splats the conf blocks into the constructors"""
     from neuraludf_b200.models import fields as F
     from neuraludf_b200.models.udf_renderer_blending import UDFRendererBlending
-    c = runner_env.ConfigFactory.parse_string(open(os.path.join(refshim.REFERENCE_ROOT, name)).read())
+    c = runner_env.ConfigFactory.parse_string(open(os.path.join(GOLDEN, name)).read())
     nerf = F.NeRF(**c["model.nerf"])
     udf = F.UDFNetwork(**c["model.udf_network"])
     var = F.SingleVarianceNetwork(**c["model.variance_network"])
@@ -69,6 +69,6 @@ def test_synthetic_dtu_layout(tmp_path):
     assert abs(np.linalg.norm(c) - 2.5) < 1e-3              # the camera sits outside the unit sphere (dataset.py:329-335)
     m = cv2.imread(os.path.join(root, "mask", "000.png"))
     assert 0.02 < (m > 0).mean() < 0.5                      # the sphere is visible and does not fill the image
-    conf = runner_env.write_conf(refshim.REFERENCE_ROOT, str(tmp_path / "t.conf"), root + "/", str(tmp_path / "exp") + "/", 3)
+    conf = runner_env.write_conf(GOLDEN, str(tmp_path / "t.conf"), root + "/", str(tmp_path / "exp") + "/", 3)
     c = runner_env.ConfigFactory.parse_string(open(conf).read())
     assert c.get_int("train.end_iter") == 3 and c.get_string("dataset.data_dir") == root + "/"
